@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                    # headline: C3, find_overlapping_iter
     python bench.py --config {C3,C3-find,C2,C4,C5} ...               # the other BASELINE.json configs
     python bench.py --impl reference [--config ...] ...              # the reference's CPU path (C port)
+    python bench.py ... --dump-outputs DIR                           # also write the last timed step's result
 
 Headline workload (BASELINE.json configs[2] with the headline iterator): a bytewise automaton of 675 000
 UniDic-like patterns; one *step* = one pass of find_overlapping_iter over a batch of 1 Mi haystacks x 4 KiB
@@ -26,6 +27,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -206,6 +208,44 @@ def mode_ids(mode_name):
             "leftmost_find_iter": (D.LEFTMOST_FIND, O.LEFTMOST_FIND)}[mode_name]
 
 
+DUMP_OFFSETS_MAX = 1 << 21       # offsets written (every k-th of them beyond that)
+DUMP_TEXT_BYTES = 8 << 20        # haystack bytes in the sample whose matches are written ...
+DUMP_HAYSTACKS_MAX = 1 << 16     # ... but no more haystacks than this
+DUMP_MATCHES_MAX = 1 << 20       # and no more match rows than this
+DUMP_SEED = 17
+
+
+def dump_outputs(out_dir, matches, offsets, hay_len):
+    """--dump-outputs: the result of one step as a caller receives it -- ``matches`` ((total, 3) int32 tensor of
+    (start, end, value)) and ``offsets`` ((n + 1,) int64 tensor) -- written to out_dir as float64 .npy files, which
+    hold every u32 position and value and every offset below 2**53 exactly.  At most about 41 MiB in all:
+
+      offsets.npy          the offsets; every k-th of them (the first included) when there are more than 2**21
+      match_haystacks.npy  a fixed, seeded sample of haystack indices (8 MiB of text, at most 65536 haystacks)
+      match_counts.npy     the number of matches of each sampled haystack
+      matches.npy          (m, 3): the sampled haystacks' matches in result order, their first 2**20 rows
+
+    The sample depends on nothing but the number of haystacks and hay_len, so two builds run with the same
+    arguments write arrays that can be compared element for element."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    o = offsets.cpu().numpy().astype(np.int64)
+    n = o.size - 1
+    stride = -(-o.size // DUMP_OFFSETS_MAX)
+    k = min(n, DUMP_HAYSTACKS_MAX, max(1, DUMP_TEXT_BYTES // max(hay_len, 1)))
+    hs = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=k, replace=False))
+    lo, counts = o[hs], o[hs + 1] - o[hs]
+    # row of every sampled match: haystack j's matches are rows lo[j] .. lo[j] + counts[j] - 1
+    firsts = np.cumsum(counts) - counts
+    rows = (np.repeat(lo - firsts, counts) + np.arange(int(counts.sum()), dtype=np.int64))[:DUMP_MATCHES_MAX]
+    m = matches.index_select(0, torch.from_numpy(rows).to(matches.device)).cpu().numpy()
+    arrays = {"offsets": o[::stride], "match_haystacks": hs, "match_counts": counts,
+              "matches": m.view(np.uint32).reshape(-1, 3)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def cpu_sample(W, opma, omode, n_hay, min_seconds, threads):
     """Times orc_bench_batch on the first n_hay haystacks of the rank's first batch: repeated until min_seconds."""
     import oracle_api as O
@@ -280,9 +320,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-overlap", action="store_true", help="one job, placement and next scan serialised (ablation)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/*.npy (float64, a seeded sample; see dump_outputs)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = CONFIGS[args.config]["steps"]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -450,6 +494,9 @@ def main():
     job_bytes = step_bytes * world
     value = job_bytes / (ms * 1e-3) / 1e9
     last_batch = (args.warmup + args.steps - 1) % len(batches)
+    if args.dump_outputs and rank == 0:
+        gm, go = group.result(last_total) if group is not None else (out_m[:last_total], out_o)
+        dump_outputs(args.dump_outputs, gm, go, hay_len)
 
     # ---- in-run parity: the result of the last timed step against the oracle -------------------------------
     # every rank scans a sample of its own shard with the oracle (counts + order-sensitive hashes per haystack,

@@ -2,7 +2,7 @@
  * dach_oracle.c -- CPU ORACLE (test infrastructure only; see dach_oracle.h).
  *
  * Plain-C restatement of daac-tools/daachorse 4.0.0.  Each function cites the
- * reference file:line (relative to /root/reference/) whose control flow it follows.
+ * reference file:line (relative to the daachorse 4.0.0 repository) whose control flow it follows.
  * V (the pattern value type) is fixed to u32.
  */
 #define _GNU_SOURCE

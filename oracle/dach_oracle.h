@@ -16,7 +16,7 @@
  * num_states doc constants, the charwise zero-length multibyte vectors, the UTF-8
  * decoder table, the mapper ranks and the serializer LE goldens.
  *
- * All file:line citations are relative to /root/reference/.
+ * All file:line citations are relative to the daachorse 4.0.0 repository.
  */
 #ifndef DACH_ORACLE_H
 #define DACH_ORACLE_H

@@ -1,21 +1,19 @@
 #!/usr/bin/env python3
 """Extract the reference's own search vectors into a JSON fixture.
 
-Reads /root/reference/tests/aho_corasick_crate_test.rs (the 136 ``SearchTest`` vectors at
-:63-382, the collections at :50-59 and the 12 test configurations at :537-645) and writes
-tests/golden/search_tests.json.  Only *data* (names, patterns, haystacks, expected
-``(value, start, end)`` triples) is extracted; no reference source code is copied.
+Reads tests/aho_corasick_crate_test.rs of a daachorse 4.0.0 checkout (the 136 ``SearchTest``
+vectors at :63-382, the collections at :50-59 and the 12 test configurations at :537-645) and
+writes tests/golden/search_tests.json.  Only *data* (names, patterns, haystacks, expected
+``(value, start, end)`` triples) is extracted; no reference source code is copied.  The tests
+read the JSON file only, so they need no copy of the crate:
 
-Run in the build container (the reference tree does not exist on the GPU box):
-
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <daachorse checkout>
 """
 import json
 import os
 import re
 import sys
 
-REF = "/root/reference/tests/aho_corasick_crate_test.rs"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "search_tests.json")
 
 GROUPS = ["BASICS", "STANDARD", "LEFTMOST", "LEFTMOST_FIRST", "LEFTMOST_LONGEST",
@@ -95,7 +93,9 @@ def parse_group(src, name):
 
 
 def main():
-    src = open(REF, encoding="utf-8").read()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    src = open(os.path.join(sys.argv[1], "tests", "aho_corasick_crate_test.rs"), encoding="utf-8").read()
     groups = {g: parse_group(src, g) for g in GROUPS}
     total = sum(len(v) for v in groups.values())
     assert total == 136, total

@@ -6,6 +6,7 @@ __graft_entry__.smoke() and by bench.py's cpu_baseline / --impl reference legs.
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -276,14 +277,17 @@ _native = None
 
 
 def native_lib():
-    """liboracle_native.so: the same source built with -march=native ON THIS BOX (the timed CPU baseline);
-    falls back to the portable build if the box has no compiler."""
+    """liboracle_native.so: the same source built with -march=native on this machine (the timed CPU baseline),
+    in a temporary directory so that the tree is not written; falls back to the portable build if the machine
+    has no compiler."""
     global _native
     if _native is None:
-        path = os.path.join(ORACLE_DIR, "liboracle_native.so")
         try:
-            subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "-B", "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-            L = C.CDLL(path)
+            with tempfile.TemporaryDirectory(prefix="dach_oracle_") as tmp:
+                path = os.path.join(tmp, "liboracle_native.so")
+                subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "native", "NATIVE_OUT=" + path],
+                                      stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+                L = C.CDLL(path)  # stays mapped after the directory is removed
         except Exception:
             L = lib()
         L.orc_bench_batch.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_void_p,

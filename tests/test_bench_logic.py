@@ -1,6 +1,6 @@
 """Host logic of bench.py that needs no GPU: the order in which a pipelined run issues scans, placements and
 finishes (a wrong order deadlocks a shard group or reuses a job that is still placing), the batch windows of every
-config, the CPU budget."""
+config, the --dump-outputs writer, the CPU budget."""
 import os
 import sys
 
@@ -66,6 +66,35 @@ def test_batch_windows_of_every_config():
         else:
             w = W(name, 10 * spec["batches"], 10)
             assert w.batch_ranges() == [(10 * k, 10 * k + 10) for k in range(spec["batches"])]
+
+
+@pytest.mark.parametrize("n,hay_len,most", [(1, 4096, 3), (300, 4096, 3), (70000, 64, 40), (3 << 20, 1 << 20, 2)])
+def test_dump_outputs(tmp_path, n, hay_len, most):
+    """--dump-outputs: float64 arrays, the sampled haystacks' matches exactly as the result holds them, the same
+    files for the same result, and the size bound however many haystacks and matches there are."""
+    import numpy as np
+    import torch
+
+    rng = np.random.default_rng(n)
+    counts = rng.integers(0, most + 1, size=n)
+    offs = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    m = torch.from_numpy(rng.integers(-2**31, 2**31, size=(int(offs[-1]), 3), dtype=np.int64).astype(np.int32))
+    o = torch.from_numpy(offs)
+    bench.dump_outputs(str(tmp_path / "a"), m, o, hay_len)
+    bench.dump_outputs(str(tmp_path / "b"), m, o, hay_len)
+    names = ["match_counts.npy", "match_haystacks.npy", "matches.npy", "offsets.npy"]
+    assert sorted(os.listdir(tmp_path / "a")) == names
+    got = {nm[:-4]: np.load(tmp_path / "a" / nm) for nm in names}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / nm)) for nm, a in zip(names, got.values()))
+    assert sum(os.path.getsize(tmp_path / "a" / nm) for nm in names) <= 64 << 20
+    stride = -(-(n + 1) // bench.DUMP_OFFSETS_MAX)
+    assert np.array_equal(got["offsets"], offs[::stride])
+    hs = got["match_haystacks"].astype(np.int64)
+    assert len(hs) == min(n, bench.DUMP_HAYSTACKS_MAX, bench.DUMP_TEXT_BYTES // hay_len)
+    assert np.all(np.diff(hs) > 0) and np.array_equal(got["match_counts"], counts[hs])
+    want = np.concatenate([m.numpy()[offs[h]: offs[h + 1]] for h in hs]).view(np.uint32)[: bench.DUMP_MATCHES_MAX]
+    assert np.array_equal(got["matches"], want)
 
 
 def test_cpu_budget_is_sane():
